@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the adjoint hot path on B200: dRdW^T*psi throughput (GCells/s) and adjoint-solve wall time.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--cells C] [--scaling weak|strong]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--cells C] [--scaling weak|strong] [--dump-outputs DIR]
 
 A "step" is one matrix-free product y = diag(n) (dR/dW)^T psi over the whole mesh (the body of the reference's GMRES
 shell-matrix callback, DASolver.C:1364-1409).  Workload: BASELINE.json configs[1], "DASimpleFoam NACA0012 SA turbulence
@@ -217,19 +217,13 @@ def run_reference(args, rank):
         return
     ni, nj = grid_for(args.cells)
     arm = CpuArm(ni * nj, "port")
-    reps = 5
-    vals, last = [], None
-    for i in range(args.warmup + max(1, args.steps)):
-        last = arm.run(reps)
-        if i >= args.warmup:
-            vals.append(last["value"])
-        if i >= args.warmup + 2:  # bounded: three timed samples
-            break
+    if args.warmup > 0:
+        arm.run(args.warmup)
+    last = arm.run(args.steps)  # one step = one product on every partition at once
     arm.close()
-    v = float(np.mean(vals))
-    last["value"] = v
+    v = last["value"]
     out = {"impl": "reference", "metric": "dRdWTPsi_GCells_per_s", "value": v, "unit": "GCells/s", "n_gpus": args.gpus,
-           "steps": len(vals), "warmup": args.warmup, "ms_per_step": 1e3 * last["seconds_per_product"], "higher_is_better": True,
+           "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * last["seconds_per_product"], "higher_is_better": True,
            "scaling": args.scaling, "vs_baseline": None, "dtype": "f64", "data": "synthetic",
            "config": {"workload": "%s NACA0012 SA %dx%dx1 O-grid, %d cells as %d partitions of %d cells on %d host cores"
                                   % (args.solver, ni, nj, ni * nj, last["cores"], last["cells_total"] // last["cores"], last["cores"])},
@@ -251,6 +245,26 @@ def emit(obj):
         sys.stdout.flush()
     else:
         os.write(_REAL_STDOUT, line)
+
+
+DUMP_BYTES = 60 << 20  # all arrays of --dump-outputs together: under 64 MB with the .npy headers
+
+
+def dump_outputs(d, arrays):
+    """Write every array as d/<name>.npy in float64, the arrays sharing DUMP_BYTES equally.  A longer array is stored as its
+    entries at np.sort(np.random.default_rng(0).choice(size, share, replace=False)): the same indices on every run of the same
+    arguments, so that two builds can be compared entry for entry."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // (8 * max(1, len(arrays)))
+    info = {}
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        size = a.size
+        if size > share:
+            a = a[np.sort(np.random.default_rng(0).choice(size, share, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+        info[name] = {"size": size, "stored": int(a.size), "sampled": size > share}
+    return {"dir": os.path.abspath(d), "arrays": info}
 
 
 def global_state(mesh, comp, U0c, thermo):
@@ -308,7 +322,14 @@ def main():
                          "(the RevB<6,7> / FwdB<6,7> kernel variants instead of the light <6,0> ones); not the default workload")
     ap.add_argument("--primal-iters", type=int, default=None,
                     help="run that many SIMPLE iterations (solvePrimal on the GPU) from the synthetic state before the adjoint legs (1 GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the run computed as DIR/<name>.npy (float64, rank 0's local vectors): dRdWTPsi, the y the last timed "
+                         "product returned, and adjoint_psi_<leg>, the solution of each adjoint-solve leg; see dump_outputs for the size bound")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -460,6 +481,7 @@ def main():
     barrier()
     e2e_s = (time.perf_counter() - t0) / args.steps
     clocks = sampler.stop() if rank == 0 else None
+    outputs = {"dRdWTPsi": y.copy()}
 
     # max over ranks
     tt = torch.tensor([ms, e2e_s * 1e3], dtype=torch.float64, device="cuda")
@@ -503,6 +525,7 @@ def main():
                            "n_matvec": st.n_matvec, "device_s": st.solve_seconds}
 
             psi_i, adjoint["idrs"] = leg("IDR(%d)" % args.idr_s, dict(kspType="idrs", idrS=args.idr_s, gmresMaxIters=3 * args.max_iters))
+            outputs["adjoint_psi_idrs"] = psi_i
             best = adjoint["idrs"]
             if not args.no_gmres and (world == 1 or args.gmres_multi):  # the GMRES leg (25 s and a 110 GB basis at 1M cells) runs on one GPU only by default
                 free_b = torch.cuda.mem_get_info()[0]
@@ -511,6 +534,7 @@ def main():
                 try:
                     psi_g, adjoint["gmres"] = leg("GMRES(%d), the reference's KSP" % restart,
                                                   dict(kspType="gmres", gmresRestart=restart, gmresMaxIters=args.max_iters))
+                    outputs["adjoint_psi_gmres"] = psi_g
                     dn = float(np.linalg.norm(psi_g))
                     adjoint["idrs"]["psi_rel_diff_vs_gmres"] = float(np.linalg.norm(psi_i - psi_g)) / dn if dn > 0 else None
                     if adjoint["gmres"]["fail"] == 0 and (best["fail"] or adjoint["gmres"]["wall_s"] < best["wall_s"]):
@@ -587,6 +611,8 @@ def main():
             arm.close()
         except Exception as e:
             out["cpu_baseline"] = {"error": str(e)}
+    if args.dump_outputs:
+        out["dumped_outputs"] = dump_outputs(args.dump_outputs, outputs)
     emit(out)
     if world > 1:
         dist.destroy_process_group()

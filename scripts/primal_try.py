@@ -1,7 +1,7 @@
 """Development driver: SIMPLE primal on a small case with the host-simulation build."""
-import sys, time
+import os, sys, time
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests.common import setup, HOSTSIM
 
 kind = sys.argv[1] if len(sys.argv) > 1 else "channel"
