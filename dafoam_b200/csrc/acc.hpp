@@ -1,13 +1,8 @@
-// Data accessors of the reverse-sweep math (rev_kernels.hpp).  The hand-derived adjoint of a cell is written once, against
-// an accessor type; two accessors exist:
-//
-//   GAcc   global SoA arrays indexed by the (rank-local) cell id -- the cell-per-thread kernels (kernel1d) used for the
-//          feature variants (MRF, patchVelocity adjoints), for polyhedral meshes whose tiles do not fit and on several GPUs
-//   TAcc*  (tile_kernels.hpp) a CTA-resident tile: the per-cell arrays of the tile and its halo rings sit in shared memory
-//          under tile-local indices, face arrays stay in global memory under global face ids
-//
-// The accessor is the only place that knows where a value lives; the arithmetic (and therefore parity with the oracle) is
-// shared.  Reference role: the CoDiPack tape evaluation inside DASolver::dRdWTMatVecMultFunction (DASolver.C:1364-1409).
+// Data accessor of the reverse-sweep math (rev_kernels.hpp).  The hand-derived adjoint of a cell (revACell / revBCell /
+// revCCell) reads and writes every value through GAcc: the global SoA arrays of the mesh, state, forward record, reverse
+// intermediates and product vector, indexed by the (rank-local) cell or face id.  GAcc is the only place that knows the
+// layout of those arrays (component strides nC or nCtot, interleaved U); the arithmetic only names values.  Reference role:
+// the CoDiPack tape evaluation inside DASolver::dRdWTMatVecMultFunction (DASolver.C:1364-1409).
 #pragma once
 #include "views.hpp"
 
@@ -92,7 +87,7 @@ struct GAcc
     DAB_HD void setYP(int c, double v) const { yP[c] = v; }
     DAB_HD void setYN(int c, double v) const { yN[c] = v; }
     DAB_HD void setYPhi(int f, double v) const { yPhi[f] = v; }
-    // ---- optional features of the cell-per-thread kernels
+    // ---- optional features: MRF zone, adjoint of the boundary reference values (patchVelocity input)
     DAB_HD bool mrfCell(int c) const { return m.mrfCell && m.mrfCell[c]; }
     DAB_HD bool bcRefOn(int pa) const { return a.bcRefb && ((a.bcMask >> pa) & 1u); }
     DAB_HD bool bcRefAny() const { return a.bcRefb != nullptr; }

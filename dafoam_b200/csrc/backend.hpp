@@ -18,30 +18,6 @@
 namespace dab
 {
 
-// L2 prefetch plan of a cell-per-thread launch (CUDA build): the CTA that processes cells [b*DAB_BLOCK, ...) first asks the
-// memory system to bring the slices of CTA b + `ahead` (about one wave of resident CTAs later) of every listed per-cell array,
-// and the owner-sorted face ranges of those cells of every listed per-face array, from HBM into L2 with bulk prefetches
-// (cp.async.bulk.prefetch.L2: one instruction per contiguous slice, no registers, no completion to wait for).  The gathers of
-// that later CTA then hit L2 (~250 cycles) instead of HBM (~800): the kernels are latency-bound, not bandwidth-bound.
-constexpr int PF_MAXC = 44, PF_MAXF = 16, PF_MAXR = 4;
-struct PfPlan
-{
-    int nC = 0, nCellArr = 0, nFaceArr = 0, ahead = 0, nChunks = 0;
-    const char* cellArr[PF_MAXC];
-    int cellBytes[PF_MAXC];
-    const char* faceArr[PF_MAXF];
-    int faceBytes[PF_MAXF];
-    const int32_t* ranges = nullptr; // [nChunks][2*PF_MAXR]: face ranges [f0, f1) owned by the cells of the chunk
-    void cell(const void* p, int bytes)
-    {
-        if (p && nCellArr < PF_MAXC) { cellArr[nCellArr] = (const char*)p; cellBytes[nCellArr++] = bytes; }
-    }
-    void face(const void* p, int bytes)
-    {
-        if (p && nFaceArr < PF_MAXF) { faceArr[nFaceArr] = (const char*)p; faceBytes[nFaceArr++] = bytes; }
-    }
-};
-
 #ifndef DAB_HOSTSIM
 #define DAB_CUDA_CHECK(x)                                                                              \
     do                                                                                                 \
@@ -68,50 +44,6 @@ __global__ void __launch_bounds__(DAB_BLOCK, LaunchTraits<F>::minBlocks) kernel1
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) f(i);
-}
-
-__device__ __forceinline__ void pfL2(const char* p, long bytes)
-{
-    if (bytes <= 0) return;
-    const unsigned long long a = (unsigned long long)p & ~15ull;
-    const unsigned long long e = ((unsigned long long)p + (unsigned long long)bytes + 15ull) & ~15ull;
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"((unsigned)(e - a)) : "memory");
-}
-
-template <class F>
-__global__ void __launch_bounds__(DAB_BLOCK, LaunchTraits<F>::minBlocks) kernel1dPf(int n, F f, PfPlan pl)
-{
-    const int ch = (int)blockIdx.x + pl.ahead;
-    if (ch < pl.nChunks)
-    {
-        const int t = (int)threadIdx.x;
-        if (t < pl.nCellArr)
-        {
-            const int c0 = ch * DAB_BLOCK;
-            const int cnt = min(DAB_BLOCK, pl.nC - c0);
-            pfL2(pl.cellArr[t] + (size_t)c0 * pl.cellBytes[t], (long)cnt * pl.cellBytes[t]);
-        }
-        else if (t >= 64 && t < 64 + pl.nFaceArr * PF_MAXR)
-        {
-            const int a = (t - 64) / PF_MAXR, r = (t - 64) % PF_MAXR;
-            const int f0 = pl.ranges[(size_t)ch * 2 * PF_MAXR + 2 * r], f1 = pl.ranges[(size_t)ch * 2 * PF_MAXR + 2 * r + 1];
-            pfL2(pl.faceArr[a] + (size_t)f0 * pl.faceBytes[a], (long)(f1 - f0) * pl.faceBytes[a]);
-        }
-    }
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) f(i);
-}
-
-// one CTA per tile (tile_kernels.hpp): the program's phases separated by block barriers, dynamic shared memory
-template <class P>
-__global__ void __launch_bounds__(P::THREADS) __maxnreg__(P::MAXREG) tileKernel(P p)
-{
-    extern __shared__ __align__(16) double dabTileSm[];
-    _Pragma("unroll") for (int ph = 0; ph < P::PHASES; ph++)
-    {
-        p.phase(ph, (int)blockIdx.x, (int)threadIdx.x, P::THREADS, dabTileSm);
-        if (ph + 1 < P::PHASES) __syncthreads();
-    }
 }
 
 struct Backend
@@ -160,47 +92,6 @@ struct Backend
         DAB_CUDA_CHECK(cudaGetLastError()); // a launch-configuration failure is not sticky: catch it here, not as wrong numbers later
         launches++;
     }
-    // cell-per-thread launch with an L2 prefetch plan (plan.ahead <= 0: one wave of resident CTAs)
-    template <class F>
-    void launchPf(int n, const F& f, PfPlan pl)
-    {
-        if (n <= 0) return;
-        if (!pl.ranges || pl.nChunks <= 0)
-        {
-            launch(n, f);
-            return;
-        }
-        static int wave = 0; // per functor type: resident CTAs of this kernel on the whole device
-        if (!wave)
-        {
-            int perSm = 0, dev = 0, sms = 0;
-            DAB_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, kernel1dPf<F>, DAB_BLOCK, 0));
-            DAB_CUDA_CHECK(cudaGetDevice(&dev));
-            DAB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-            wave = std::max(1, perSm * sms);
-        }
-        if (pl.ahead <= 0) pl.ahead = wave;
-        const int bs = DAB_BLOCK;
-        kernel1dPf<F><<<(n + bs - 1) / bs, bs, 0, stream>>>(n, f, pl);
-        DAB_CUDA_CHECK(cudaGetLastError());
-        launches++;
-    }
-    template <class P>
-    void launchTiles(int nTiles, const P& p)
-    {
-        if (nTiles <= 0) return;
-        static bool configured = false; // per program type: opt in to > 48 KB of dynamic shared memory
-        const int bytes = P::SM_DOUBLES * (int)sizeof(double);
-        if (!configured)
-        {
-            DAB_CUDA_CHECK(cudaFuncSetAttribute(tileKernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-            DAB_CUDA_CHECK(cudaFuncSetAttribute(tileKernel<P>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            configured = true;
-        }
-        tileKernel<P><<<nTiles, P::THREADS, bytes, stream>>>(p);
-        DAB_CUDA_CHECK(cudaGetLastError());
-        launches++;
-    }
     // CUDA-event timer on the solver's stream
     struct Timer
     {
@@ -238,17 +129,6 @@ struct Backend
     void launch(int n, const F& f)
     {
         for (int i = 0; i < n; i++) f(i);
-        launches++;
-    }
-    template <class F>
-    void launchPf(int n, const F& f, const PfPlan&) { launch(n, f); }
-    // test-only emulation of a tile launch: tile by tile, phase by phase, one "thread" walking the whole CTA's work
-    template <class P>
-    void launchTiles(int nTiles, const P& p)
-    {
-        std::vector<double> sm((size_t)P::SM_DOUBLES, 0.0);
-        for (int t = 0; t < nTiles; t++)
-            for (int ph = 0; ph < P::PHASES; ph++) p.phase(ph, t, 0, 1, sm.data());
         launches++;
     }
     struct Timer

@@ -143,12 +143,12 @@ DAB_HD FaceRef faceOfE2(int nIF, int e, int n)
 }
 #define DAB_ACC_FACES(NF)                                        \
     int e_[(NF) > 0 ? (NF) : 1], n_[(NF) > 0 ? (NF) : 1];        \
-    if constexpr ((NF) > 0) A.template faceRow<((NF) > 0 ? (NF) : 1)>(c, e_, n_);
+    if constexpr ((NF) > 0) A.faceRow<((NF) > 0 ? (NF) : 1)>(c, e_, n_);
 #define DAB_ACC_FACE(NF, k) ((NF) > 0 ? faceOfE2(A.nIF(), e_[(NF) > 0 ? (k) : 0], n_[(NF) > 0 ? (k) : 0]) : A.face(c, k))
 
 // RevA of one cell: adjoint of FwdC + cell-level adjoint of the momentum row
-template <int NF, class Acc>
-DAB_HD void revACell(const Acc& A, const Params& q, int c)
+template <int NF>
+DAB_HD void revACell(const GAcc& A, const Params& q, int c)
 {
     const double Uc[3] = {A.U(c, 0), A.U(c, 1), A.U(c, 2)};
     const double V = A.V(c);
@@ -273,9 +273,9 @@ struct RevA
 
 // RevB of one cell.  FEAT: bit 0 = linearUpwindV limiter compiled in, bit 1 = wall-function nut BC compiled in, bit 2 = adjoint of
 // the boundary reference values (patchVelocity input) compiled in (the common configuration without them keeps its register
-// budget).  gradOnly (tile kernels, halo ring): only the adjoints of grad(U) / grad(nuTilda) are stored.
-template <int NF, int FEAT, class Acc>
-DAB_HD void revBCell(const Acc& A, const Params& q, int c, bool gradOnly)
+// budget).
+template <int NF, int FEAT>
+DAB_HD void revBCell(const GAcc& A, const Params& q, int c)
 {
     const int schU = q.divU, schN = q.divNut;
     const double Uc[3] = {A.U(c, 0), A.U(c, 1), A.U(c, 2)};
@@ -545,23 +545,17 @@ DAB_HD void revBCell(const Acc& A, const Params& q, int c, bool gradOnly)
             }
             phib_acc += mb;
         }
-        if (!gradOnly)
-        {
-            if (fr.s > 0)
-                A.setYPhi(f, (phib_acc - (q.nrPhi ? rmS : 1.0) * xphif) * phiRowScale(q, mS));
-            else if (A.ghost(fr.n))
-                A.setYPhi(f, 0.0); // cut face whose phi belongs to the neighbouring rank
-        }
+        if (fr.s > 0)
+            A.setYPhi(f, (phib_acc - (q.nrPhi ? rmS : 1.0) * xphif) * phiRowScale(q, mS));
+        else if (A.ghost(fr.n))
+            A.setYPhi(f, 0.0); // cut face whose phi belongs to the neighbouring rank
     }
     if (q.turb) saSourceAdj(ntc, q.nu, A.yWall(c), gUc, gNc, zc, nt2, gUb, gNb, q.saFv3);
-    if (!gradOnly)
-    {
-        for (int j = 0; j < 3; j++) A.setU2(c, j, U2[j]);
-        if ((FEAT & 4) && A.bcRefAny())
-            for (int j = 0; j < 3; j++) A.addBcRef(c, j, refb[j]);
-        A.setNt2(c, nt2);
-        A.setNutb(c, nuEb);
-    }
+    for (int j = 0; j < 3; j++) A.setU2(c, j, U2[j]);
+    if ((FEAT & 4) && A.bcRefAny())
+        for (int j = 0; j < 3; j++) A.addBcRef(c, j, refb[j]);
+    A.setNt2(c, nt2);
+    A.setNutb(c, nuEb);
     for (int i = 0; i < 9; i++) A.setGUb(c, i, gUb[i]);
     for (int i = 0; i < 3; i++) A.setGNtb(c, i, gNb[i]);
 }
@@ -579,13 +573,13 @@ struct RevB
     DAB_HD void operator()(int c) const
     {
         const GAcc A{m, s, r, a, x, nullptr, nullptr, nullptr, y + (size_t)(q.turb ? 5 : 4) * m.nC};
-        revBCell<NF, FEAT>(A, q, c, false);
+        revBCell<NF, FEAT>(A, q, c);
     }
 };
 
 // RevC of one cell: adjoint of FwdA (Gauss-gradient transpose, nut(nuTilda), BC adjoints) + final sum and state scaling
-template <int NF, class Acc>
-DAB_HD void revCCell(const Acc& A, const Params& q, int c, int functionMode)
+template <int NF>
+DAB_HD void revCCell(const GAcc& A, const Params& q, int c, int functionMode)
 {
     const double iVc = frcp(A.V(c));
     double Ub[3], pb = A.pdir(c), nb = 0.0;

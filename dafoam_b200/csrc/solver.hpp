@@ -13,7 +13,6 @@
 #include "views.hpp"
 #include "fwd_kernels.hpp"
 #include "rev_kernels.hpp"
-#include "tile_kernels.hpp"
 #include "comp_kernels.hpp"
 #include "comp_rev_kernels.hpp"
 #include "krylov.hpp"
@@ -72,80 +71,6 @@ template <int NF> struct LaunchTraits<cRevC<NF>> { static constexpr int minBlock
 template <int NF> struct LaunchTraits<cFwdE<NF>> { static constexpr int minBlocks = 4; };
 template <int NF> struct LaunchTraits<cFwdC<NF>> { static constexpr int minBlocks = 4; };
 #endif
-
-// optional-feature dispatch for the two heavy kernels (hex meshes: 4 variants; other meshes: the full-featured one)
-#define DAB_LAUNCH_NFF(n, F, ...)                                     \
-    do                                                                \
-    {                                                                 \
-        if (hex6)                                            \
-        {                                                             \
-            switch (featureMask())                                    \
-            {                                                         \
-            case 0: be.launch(n, F<6, 0>{__VA_ARGS__}); break;        \
-            case 1: be.launch(n, F<6, 1>{__VA_ARGS__}); break;        \
-            case 2: be.launch(n, F<6, 2>{__VA_ARGS__}); break;        \
-            case 3: be.launch(n, F<6, 3>{__VA_ARGS__}); break;        \
-            default: be.launch(n, F<6, 7>{__VA_ARGS__}); break;       \
-            }                                                         \
-        }                                                             \
-        else be.launch(n, F<0, 7>{__VA_ARGS__});                      \
-    } while (0)
-
-// the same launches over the cell range [c0, c0 + n) (interior / cut-adjacent split for communication overlap)
-#define DAB_LAUNCH_NF_R(c0, n, F, ...)                                                      \
-    do                                                                                      \
-    {                                                                                       \
-        if (hex6) be.launch(n, Shifted<F<6>>{F<6>{__VA_ARGS__}, c0});              \
-        else be.launch(n, Shifted<F<0>>{F<0>{__VA_ARGS__}, c0});                            \
-    } while (0)
-#define DAB_LAUNCH_NFF_R(c0, n, F, ...)                                                     \
-    do                                                                                      \
-    {                                                                                       \
-        if (hex6)                                                                  \
-        {                                                                                   \
-            switch (featureMask())                                                          \
-            {                                                                               \
-            case 0: be.launch(n, Shifted<F<6, 0>>{F<6, 0>{__VA_ARGS__}, c0}); break;        \
-            case 1: be.launch(n, Shifted<F<6, 1>>{F<6, 1>{__VA_ARGS__}, c0}); break;        \
-            case 2: be.launch(n, Shifted<F<6, 2>>{F<6, 2>{__VA_ARGS__}, c0}); break;        \
-            case 3: be.launch(n, Shifted<F<6, 3>>{F<6, 3>{__VA_ARGS__}, c0}); break;        \
-            default: be.launch(n, Shifted<F<6, 7>>{F<6, 7>{__VA_ARGS__}, c0}); break;       \
-            }                                                                               \
-        }                                                                                   \
-        else be.launch(n, Shifted<F<0, 7>>{F<0, 7>{__VA_ARGS__}, c0});                      \
-    } while (0)
-
-// hexahedral meshes (6 faces per cell) get fully unrolled face loops; anything else the run-time loop
-#define DAB_LAUNCH_NF(n, F, ...)                                  \
-    do                                                            \
-    {                                                             \
-        if (hex6) be.launch(n, F<6>{__VA_ARGS__});       \
-        else be.launch(n, F<0>{__VA_ARGS__});                     \
-    } while (0)
-
-// the same with an L2 prefetch plan (backend.hpp PfPlan)
-#define DAB_LAUNCH_NF_PF(pl, n, F, ...)                           \
-    do                                                            \
-    {                                                             \
-        if (hex6) be.launchPf(n, F<6>{__VA_ARGS__}, pl);          \
-        else be.launchPf(n, F<0>{__VA_ARGS__}, pl);               \
-    } while (0)
-#define DAB_LAUNCH_NFF_PF(pl, n, F, ...)                                  \
-    do                                                                    \
-    {                                                                     \
-        if (hex6)                                                         \
-        {                                                                 \
-            switch (featureMask())                                        \
-            {                                                             \
-            case 0: be.launchPf(n, F<6, 0>{__VA_ARGS__}, pl); break;      \
-            case 1: be.launchPf(n, F<6, 1>{__VA_ARGS__}, pl); break;      \
-            case 2: be.launchPf(n, F<6, 2>{__VA_ARGS__}, pl); break;      \
-            case 3: be.launchPf(n, F<6, 3>{__VA_ARGS__}, pl); break;      \
-            default: be.launchPf(n, F<6, 7>{__VA_ARGS__}, pl); break;     \
-            }                                                             \
-        }                                                                 \
-        else be.launchPf(n, F<0, 7>{__VA_ARGS__}, pl);                    \
-    } while (0)
 
 // DAInputPatchVelocity (reference src/adjoint/DAInput/DAInputPatchVelocity.C): input = (|U|, angle of attack in degrees)
 struct PatchVelocityDef
@@ -269,18 +194,6 @@ struct Solver
     Partition part;
     DevBuf<double> psiP, psiN, psiPhi, psiT; // working copies of the input vector with ghost slots (multi-rank only)
 
-    // CTA-resident product kernels (tile_kernels.hpp): one GPU, DASimpleFoam without an MRF zone
-    TileMap tiles;
-    DevBuf<int32_t> dTileCum, dTileGid, dTileTf, dTileTn;
-    TileView tvw{};
-    bool tilesOn = false;
-    int tileCellsHint = 0; // adjEqnOption.tileCells (extension): cells per tile of a tile-major numbered mesh; 0 = search
-
-    // L2 prefetch plans of the cell-per-thread product kernels (backend.hpp PfPlan)
-    DevBuf<int32_t> dPfRanges;
-    int pfChunks = 0;
-    bool pfOn = false;
-
     bool fvSourceDirty = false;
     bool hex6 = false; // every owned cell has exactly 6 faces: the kernels with fully unrolled, break-free face loops apply
     int nCellStates() const { return 4 + (par.comp ? 1 : 0) + (par.turb ? 1 : 0); }
@@ -299,6 +212,57 @@ struct Solver
                 if (par.bcKind[F_NUT][p] == BC_NUT_SPALDING) f |= 2;
         if (av.bcRefb) f = 7; // patchVelocity product: the full-featured variant also carries the BC-reference adjoint
         return f;
+    }
+
+    // launch F<NF>{a...} over the cells [0, n): hexahedral meshes (6 faces per cell) get fully unrolled face loops (NF = 6),
+    // anything else the run-time loop (NF = 0)
+    template <template <int> class F, class... A>
+    void launchNF(int n, const A&... a)
+    {
+        if (hex6) be.launch(n, F<6>{a...});
+        else be.launch(n, F<0>{a...});
+    }
+    // the same with the optional-feature dispatch of the two heavy kernels (hex meshes: 4 variants; other meshes: the full-featured one)
+    template <template <int, int> class F, class... A>
+    void launchNFF(int n, const A&... a)
+    {
+        if (!hex6)
+        {
+            be.launch(n, F<0, 7>{a...});
+            return;
+        }
+        switch (featureMask())
+        {
+        case 0: be.launch(n, F<6, 0>{a...}); break;
+        case 1: be.launch(n, F<6, 1>{a...}); break;
+        case 2: be.launch(n, F<6, 2>{a...}); break;
+        case 3: be.launch(n, F<6, 3>{a...}); break;
+        default: be.launch(n, F<6, 7>{a...}); break;
+        }
+    }
+    // the same launches over the cell range [c0, c0 + n) (interior / cut-adjacent split for communication overlap)
+    template <template <int> class F, class... A>
+    void launchNFRange(int c0, int n, const A&... a)
+    {
+        if (hex6) be.launch(n, Shifted<F<6>>{F<6>{a...}, c0});
+        else be.launch(n, Shifted<F<0>>{F<0>{a...}, c0});
+    }
+    template <template <int, int> class F, class... A>
+    void launchNFFRange(int c0, int n, const A&... a)
+    {
+        if (!hex6)
+        {
+            be.launch(n, Shifted<F<0, 7>>{F<0, 7>{a...}, c0});
+            return;
+        }
+        switch (featureMask())
+        {
+        case 0: be.launch(n, Shifted<F<6, 0>>{F<6, 0>{a...}, c0}); break;
+        case 1: be.launch(n, Shifted<F<6, 1>>{F<6, 1>{a...}, c0}); break;
+        case 2: be.launch(n, Shifted<F<6, 2>>{F<6, 2>{a...}, c0}); break;
+        case 3: be.launch(n, Shifted<F<6, 3>>{F<6, 3>{a...}, c0}); break;
+        default: be.launch(n, Shifted<F<6, 7>>{F<6, 7>{a...}, c0}); break;
+        }
     }
 
     // ------------------------------------------------------------------------------------------
@@ -382,7 +346,7 @@ struct Solver
         lap("dictionaries");
         applyOptions(optionsJson, true);
         upload();
-        lap("upload + tile/prefetch maps");
+        lap("upload");
         initialStates(caseDir);
         lap("initial states");
     }
@@ -706,7 +670,6 @@ struct Solver
             fpRelTol = a->numOr("fpRelTol", fpRelTol);
             fpMinResTolDiff = a->numOr("fpMinResTolDiff", fpMinResTolDiff);
             fpOmega = a->numOr("fpOmega", fpOmega);
-            tileCellsHint = (int)a->numOr("tileCells", tileCellsHint);
             {
                 const int sa = (int)a->numOr("coarseSparseAP", coarseSparseAP);
                 if (sa != coarseSparseAP) { coarseSparseAP = sa; kry.pcValid = false; }
@@ -1028,7 +991,7 @@ struct Solver
         dOwn.upload(be, hm.own);
         dNei.upload(be, hm.nei);
         dCellFaces.upload(be, hm.cellFaces);
-        hex6 = hm.maxCF == 6 && !(getenv("DAB_NOHEX6") && atoi(getenv("DAB_NOHEX6")) > 0); // DAB_NOHEX6: measurement hook (rolled face loops)
+        hex6 = hm.maxCF == 6;
         for (size_t i = 0; i < hm.cellFaces.size() && hex6; i++)
             if (hm.cellFaces[i] < 0) hex6 = false;
         hm.buildCellNbr();
@@ -1099,164 +1062,6 @@ struct Solver
             av.cHe = aCHe.p; av.cEk = aCEk.p;
         }
         dR.alloc(be, nd); dX.alloc(be, nd); dY2.alloc(be, nd);
-        setupTiles();
-        setupPrefetch();
-    }
-
-    // choose a tile size whose tiles (with two halo rings) fit the capacities compiled into tile_kernels.hpp and build the tile map
-    void setupTiles()
-    {
-        tilesOn = false;
-        // measured on B200 (profiles/r02_tile_kernels.md): the tile kernels are slower than the cell-per-thread kernels (face data
-        // still comes from global memory, one or two CTAs per SM) -- they stay a tested option (DAB_TILE=1), not the default
-        const char* env = getenv("DAB_TILE");
-        if (!env || atoi(env) == 0) return;
-        if (partitioned || par.comp || mrf.on || hm.nC < 64) return;
-        std::vector<int> cand;
-        if (tileCellsHint > 0) cand.push_back(tileCellsHint);
-        for (int t : {192, 176, 168, 160, 144, 128, 112, 96, 80, 64, 48, 32}) cand.push_back(t);
-        int best = 0;
-        double bestRatio = 1e30;
-        for (int T : cand)
-        {
-            if (T > TILE_TMAX || T < 1) continue;
-            int maxRun, maxAll;
-            long sumAll;
-            TileMap::measure(hm, T, 2, maxRun, maxAll, sumAll);
-            if (maxRun > TILE_EXT1 || maxAll > TILE_EXT2) continue;
-            const double ratio = (double)sumAll / hm.nC;
-            if (ratio < bestRatio)
-            {
-                bestRatio = ratio;
-                best = T;
-            }
-            if (T == tileCellsHint && ratio < 1.8) break; // the caller's hint fits and is compact
-        }
-        if (!best) return;
-        tiles.build(hm, best, 2);
-        dTileCum.upload(be, tiles.cum);
-        dTileGid.upload(be, tiles.gid);
-        dTileTf.upload(be, tiles.tf);
-        dTileTn.upload(be, tiles.tn);
-        tvw.T = tiles.T; tvw.nTiles = tiles.nTiles; tvw.R = tiles.R; tvw.maxCF = tiles.maxCF; tvw.ln = tiles.ln; tvw.ls = tiles.ls;
-        tvw.cum = dTileCum.p; tvw.gid = dTileGid.p; tvw.tf = dTileTf.p; tvw.tn = dTileTn.p;
-        tilesOn = true;
-        if (printInfo || getenv("DAB_TILE_INFO"))
-            fprintf(stderr, "[dab200] tiles: %d cells per tile, %d tiles, local cells per owned cell %.3f (ring 1: %.3f), max %d / %d\n", tiles.T,
-                    tiles.nTiles, bestRatio, (double)tiles.sumRun / hm.nC, tiles.maxRun, tiles.maxAll);
-    }
-
-    // face ranges owned by each chunk of DAB_BLOCK consecutive cells: OpenFOAM orders internal faces by owner, so the faces a
-    // chunk owns are one contiguous range; boundary faces are contiguous per patch when the patch is ordered by owner cell
-    void setupPrefetch()
-    {
-        pfOn = false;
-#ifndef DAB_HOSTSIM
-        // measured on B200 (profiles/r02_kernel_experiments.md, #5): 2-17 % SLOWER at every prefetch distance -- the plans stay an
-        // opt-in measurement hook (DAB_PREFETCH_L2=1), not the default
-        const char* env = getenv("DAB_PREFETCH_L2");
-        if (!env || atoi(env) == 0) return;
-        const int nC = hm.nC, nIF = hm.nIF;
-        for (int f = 1; f < nIF; f++)
-            if (hm.own[f] < hm.own[f - 1]) return; // not in upper-triangular order: no plan
-        const int bs = DAB_BLOCK;
-        pfChunks = (nC + bs - 1) / bs;
-        std::vector<int32_t> rg((size_t)pfChunks * 2 * PF_MAXR, 0);
-        // patches whose faces are sorted by owner
-        std::vector<int> sortedPatch;
-        for (size_t p = 0; p < hm.patches.size(); p++)
-        {
-            bool ok = hm.patches[p].size > 0;
-            for (int i = 1; i < hm.patches[p].size && ok; i++)
-                if (hm.own[hm.patches[p].start + i] < hm.own[hm.patches[p].start + i - 1]) ok = false;
-            if (ok) sortedPatch.push_back((int)p);
-        }
-        auto lower = [&](int a, int b, int c) { return (int)(std::lower_bound(hm.own.begin() + a, hm.own.begin() + b, c) - hm.own.begin()); };
-        for (int k = 0; k < pfChunks; k++)
-        {
-            const int c0 = k * bs, c1 = std::min(nC, c0 + bs);
-            int nr = 0;
-            int32_t* r = &rg[(size_t)k * 2 * PF_MAXR];
-            r[0] = lower(0, nIF, c0);
-            r[1] = lower(0, nIF, c1);
-            nr = 1;
-            for (int p : sortedPatch)
-            {
-                if (nr >= PF_MAXR) break;
-                const int a = hm.patches[p].start, b = a + hm.patches[p].size;
-                const int f0 = lower(a, b, c0), f1 = lower(a, b, c1);
-                if (f1 > f0)
-                {
-                    r[2 * nr] = f0;
-                    r[2 * nr + 1] = f1;
-                    nr++;
-                }
-            }
-        }
-        dPfRanges.upload(be, rg);
-        pfOn = true;
-#endif
-    }
-    PfPlan pfBase() const
-    {
-        PfPlan pl;
-        if (!pfOn) return pl;
-        pl.nC = hm.nC;
-        pl.nChunks = pfChunks;
-        pl.ranges = dPfRanges.p;
-        static const int ahead = getenv("DAB_PF_AHEAD") ? atoi(getenv("DAB_PF_AHEAD")) : 0;
-        pl.ahead = ahead;
-        const size_t nC = hm.nC;
-        for (int k = 0; k < hm.maxCF && k < 6; k++)
-        {
-            pl.cell(mv.cellFaces + (size_t)k * nC, 4);
-            pl.cell(mv.cellNbr + (size_t)k * nC, 4);
-        }
-        return pl;
-    }
-    PfPlan pfRevA(const PsiView& pv) const
-    {
-        PfPlan pl = pfBase();
-        if (!pfOn) return pl;
-        const size_t nT = hm.nCtot;
-        pl.cell(sv.U, 24); pl.cell(pv.U, 24); pl.cell(pv.p, 8); pl.cell(mv.V, 8); pl.cell(sv.p, 8); pl.cell(rv.rAU, 8); pl.cell(rv.D0, 8);
-        for (int j = 0; j < 3; j++) { pl.cell(rv.gP + j * nT, 8); pl.cell(rv.HbyA + j * nT, 8); }
-        pl.face(mv.magSf, 8); pl.face(mv.delta, 8); pl.face(mv.Sx, 8); pl.face(mv.Sy, 8); pl.face(mv.Sz, 8); pl.face(pv.phi, 8);
-        pl.face(mv.w, 8); pl.face(mv.kx, 8); pl.face(mv.ky, 8); pl.face(mv.kz, 8); pl.face(sv.phi, 8);
-        return pl;
-    }
-    PfPlan pfRevB(const PsiView& pv) const
-    {
-        PfPlan pl = pfBase();
-        if (!pfOn) return pl;
-        const size_t nT = hm.nCtot;
-        pl.cell(sv.U, 24); pl.cell(rv.nut, 8); pl.cell(mv.V, 8); pl.cell(av.Dn, 8); pl.cell(rv.flag, 8);
-        for (int i = 0; i < 9; i++) pl.cell(rv.gU + i * nT, 8);
-        for (int j = 0; j < 3; j++) { pl.cell(av.mt + j * nT, 8); pl.cell((j == 0 ? mv.Cx : (j == 1 ? mv.Cy : mv.Cz)), 8); }
-        if (par.turb)
-        {
-            pl.cell(sv.nt, 8); pl.cell(pv.nt, 8); pl.cell(mv.yWall, 8);
-            for (int j = 0; j < 3; j++) pl.cell(rv.gNt + j * nT, 8);
-        }
-        pl.face(sv.phi, 8); pl.face(mv.Sx, 8); pl.face(mv.Sy, 8); pl.face(mv.Sz, 8); pl.face(mv.magSf, 8); pl.face(mv.delta, 8); pl.face(mv.w, 8);
-        pl.face(mv.kx, 8); pl.face(mv.ky, 8); pl.face(mv.kz, 8); pl.face(mv.Cfx, 8); pl.face(mv.Cfy, 8); pl.face(mv.Cfz, 8); pl.face(pv.phi, 8);
-        return pl;
-    }
-    PfPlan pfRevC() const
-    {
-        PfPlan pl = pfBase();
-        if (!pfOn) return pl;
-        const size_t nT = hm.nCtot, nC = hm.nC;
-        pl.cell(av.pdir, 8); pl.cell(mv.V, 8);
-        for (int j = 0; j < 3; j++) { pl.cell(av.Udir + j * nC, 8); pl.cell(av.U2 + j * nC, 8); pl.cell(av.gPb + j * nT, 8); }
-        for (int i = 0; i < 9; i++) pl.cell(av.gUb + i * nT, 8);
-        if (par.turb)
-        {
-            pl.cell(av.nt2, 8); pl.cell(av.nutb, 8); pl.cell(sv.nt, 8);
-            for (int j = 0; j < 3; j++) pl.cell(av.gNtb + j * nT, 8);
-        }
-        pl.face(mv.Sx, 8); pl.face(mv.Sy, 8); pl.face(mv.Sz, 8); pl.face(mv.w, 8); pl.face(sv.phi, 8); pl.face(mv.delta, 8); pl.face(mv.magSf, 8);
-        return pl;
     }
 
     // DASolver::calcPCMatWithFvMatrix(PCMat, turbOnly = 1) (reference DASolver.C:2888-2988 + DASpalartAllmaras::getFvMatrixFields,
@@ -1282,7 +1087,7 @@ struct Solver
         EqnView e{nC, mcf, 1, off.p, diag.p, b.p, mv.cellNbr};
         Params pq = par;
         pq.divNut = DIV_UPWIND; // "div(pc)"
-        DAB_LAUNCH_NF(nC, NutEqnAssemble, mv, pq, sv, rv, e, primal.alphaN);
+        launchNF<NutEqnAssemble>(nC, mv, pq, sv, rv, e, primal.alphaN);
         std::vector<double> hOff((size_t)mcf * nC), hD(nC);
         be.d2h(hOff.data(), off.p, hOff.size() * sizeof(double));
         be.d2h(hD.data(), diag.p, hD.size() * sizeof(double));
@@ -1308,27 +1113,6 @@ struct Solver
                 cols.push_back(base + c);
                 vals.push_back(hOff[(size_t)k * nC + c] * par.sNut / resScale(c));
             }
-    }
-
-    bool tileProduct() const { return tilesOn && av.bcRefb == nullptr; }
-    void launchTileA(const PsiView& pv)
-    {
-        if (hex6) be.launchTiles(tvw.nTiles, ProdTileA<6>{mv, par, sv, rv, av, pv, tvw});
-        else be.launchTiles(tvw.nTiles, ProdTileA<0>{mv, par, sv, rv, av, pv, tvw});
-    }
-    void launchTileBC(const PsiView& pv, double* y)
-    {
-        if (hex6)
-        {
-            switch (featureMask())
-            {
-            case 0: be.launchTiles(tvw.nTiles, ProdTileBC<6, 0>{mv, par, sv, rv, av, pv, y, tvw}); break;
-            case 1: be.launchTiles(tvw.nTiles, ProdTileBC<6, 1>{mv, par, sv, rv, av, pv, y, tvw}); break;
-            case 2: be.launchTiles(tvw.nTiles, ProdTileBC<6, 2>{mv, par, sv, rv, av, pv, y, tvw}); break;
-            default: be.launchTiles(tvw.nTiles, ProdTileBC<6, 3>{mv, par, sv, rv, av, pv, y, tvw}); break;
-            }
-        }
-        else be.launchTiles(tvw.nTiles, ProdTileBC<0, 3>{mv, par, sv, rv, av, pv, y, tvw});
     }
 
     // initial states from the 0/ files (DASimpleFoam::initSolver createFieldsSimple.H role); phi = linear-interpolated U . Sf
@@ -1575,37 +1359,37 @@ struct Solver
         if (par.comp)
         {
             // DARhoSimpleFoam: closures + gradients, momentum/SA rows, energy row, pressure/flux rows (comp_kernels.hpp)
-            DAB_LAUNCH_NF(hm.nCtot, cFwdA, mv, par, sv, rv); // closures of the ghost cells come from their exchanged states
+            launchNF<cFwdA>(hm.nCtot, mv, par, sv, rv); // closures of the ghost cells come from their exchanged states
             if (exchange && ghosted())
             {
                 std::vector<HaloItem> it{{rv.gU, 9, 1, nT}, {rv.gP, 3, 1, nT}, {rv.gHe, 3, 1, nT}};
                 if (par.turb) it.push_back({rv.gNt, 3, 1, nT});
                 halo.exchangeCells(it);
             }
-            DAB_LAUNCH_NF(hm.nC, cFwdB, mv, par, sv, rv, isPC, Rdev);
-            DAB_LAUNCH_NF(hm.nC, cFwdE, mv, par, sv, rv, isPC, Rdev);
+            launchNF<cFwdB>(hm.nC, mv, par, sv, rv, isPC, Rdev);
+            launchNF<cFwdE>(hm.nC, mv, par, sv, rv, isPC, Rdev);
             if (exchange && ghosted()) halo.exchangeCells({{rv.rAU, 1, 1, nT}, {rv.HbyA, 3, 1, nT}, {rv.flag, 1, 1, nT}});
             if (isPC && par.transonic)
             {
                 Params pq = par; // div(pc) scheme and transonicPCOption for the preconditioner residual
                 pq.divPhidP = DIV_UPWIND;
                 pq.transonic = transonicPCOption == 1 ? 2 : (transonicPCOption == 2 ? 3 : 1);
-                DAB_LAUNCH_NF(hm.nC, cFwdC, mv, pq, sv, rv, Rdev);
+                launchNF<cFwdC>(hm.nC, mv, pq, sv, rv, Rdev);
             }
             else
-                DAB_LAUNCH_NF(hm.nC, cFwdC, mv, par, sv, rv, Rdev);
+                launchNF<cFwdC>(hm.nC, mv, par, sv, rv, Rdev);
             return;
         }
-        DAB_LAUNCH_NF(hm.nCtot, FwdA, mv, par, sv, rv);
+        launchNF<FwdA>(hm.nCtot, mv, par, sv, rv);
         if (exchange && ghosted())
         {
             std::vector<HaloItem> it{{rv.gU, 9, 1, nT}, {rv.gP, 3, 1, nT}};
             if (par.turb) it.push_back({rv.gNt, 3, 1, nT});
             halo.exchangeCells(it);
         }
-        DAB_LAUNCH_NFF(hm.nC, FwdB, mv, par, sv, rv, isPC, Rdev);
+        launchNFF<FwdB>(hm.nC, mv, par, sv, rv, isPC, Rdev);
         if (exchange && ghosted()) halo.exchangeCells({{rv.rAU, 1, 1, nT}, {rv.HbyA, 3, 1, nT}, {rv.flag, 1, 1, nT}});
-        DAB_LAUNCH_NF(hm.nC, FwdC, mv, par, sv, rv, Rdev);
+        launchNF<FwdC>(hm.nC, mv, par, sv, rv, Rdev);
     }
 
     void ensureRecorded()
@@ -1621,9 +1405,6 @@ struct Solver
         recorded = (isPC == 0);
         be.d2h(R, dR.p, (size_t)nDof() * sizeof(double));
     }
-
-    // y = diag(n) (dR/dW)^T x on device vectors (external layout)
-    void launchRevA(const PsiView& pv) { DAB_LAUNCH_NF(hm.nC, RevA, mv, par, sv, rv, av, pv); }
 
     PsiView psiView(const double* x)
     {
@@ -1669,6 +1450,7 @@ struct Solver
         return v;
     }
 
+    // y = diag(n) (dR/dW)^T x on device vectors (external layout)
     void matVecDev(const double* x, double* y)
     {
         ensureRecorded();
@@ -1677,53 +1459,47 @@ struct Solver
             // DARhoSimpleFoam reverse sweep (comp_rev_kernels.hpp), one GPU
             const PsiView pv = psiView(x);
             const int nTc = hm.nCtot;
-            DAB_LAUNCH_NF(hm.nC, cRevA, mv, par, sv, rv, av, pv);
+            launchNF<cRevA>(hm.nC, mv, par, sv, rv, av, pv);
             if (ghosted()) halo.exchangeCells({{av.mt, 3, 1, nTc}, {av.Dn, 1, 1, nTc}, {av.gPb, 3, 1, nTc}});
-            DAB_LAUNCH_NF(hm.nC, cRevB, mv, par, sv, rv, av, pv, y);
-            DAB_LAUNCH_NF(hm.nC, cRevE, mv, par, sv, rv, av, pv, y);
+            launchNF<cRevB>(hm.nC, mv, par, sv, rv, av, pv, y);
+            launchNF<cRevE>(hm.nC, mv, par, sv, rv, av, pv, y);
             if (ghosted())
             {
                 std::vector<HaloItem> it{{av.gUb, 9, 1, nTc}, {av.gHeb, 3, 1, nTc}};
                 if (par.turb) it.push_back({av.gNtb, 3, 1, nTc});
                 halo.exchangeCells(it);
             }
-            DAB_LAUNCH_NF(hm.nC, cRevC, mv, par, sv, rv, av, y);
+            launchNF<cRevC>(hm.nC, mv, par, sv, rv, av, y);
             return;
         }
         const int nT = hm.nCtot;
         if (!ghosted())
         {
             const PsiView pv = psiView(x);
-            if (tileProduct())
-            {
-                launchTileA(pv);
-                launchTileBC(pv, y);
-                return;
-            }
-            DAB_LAUNCH_NF_PF(pfRevA(pv), hm.nC, RevA, mv, par, sv, rv, av, pv);
-            DAB_LAUNCH_NFF_PF(pfRevB(pv), hm.nC, RevB, mv, par, sv, rv, av, pv, y);
-            DAB_LAUNCH_NF_PF(pfRevC(), hm.nC, RevC, mv, par, sv, rv, av, y, 0);
+            launchNF<RevA>(hm.nC, mv, par, sv, rv, av, pv);
+            launchNFF<RevB>(hm.nC, mv, par, sv, rv, av, pv, y);
+            launchNF<RevC>(hm.nC, mv, par, sv, rv, av, y, 0);
             return;
         }
         // several ranks: every ghost exchange runs on the communication stream while the interior cells (no neighbour on
         // another rank) of the next stage are processed; the cut-adjacent cells follow once the ghosts have arrived
         const int nI = hm.nInterior < 0 ? hm.nC : hm.nInterior, nB = hm.nC - nI;
         const PsiView pv = psiViewStart(x);
-        DAB_LAUNCH_NF_R(0, nI, RevA, mv, par, sv, rv, av, pv);
+        launchNFRange<RevA>(0, nI, mv, par, sv, rv, av, pv);
         halo.finish();
-        DAB_LAUNCH_NF_R(nI, nB, RevA, mv, par, sv, rv, av, pv);
+        launchNFRange<RevA>(nI, nB, mv, par, sv, rv, av, pv);
         halo.start(halo.cells, {{av.mt, 3, 1, nT}, {av.Dn, 1, 1, nT}, {av.gPb, 3, 1, nT}});
-        DAB_LAUNCH_NFF_R(0, nI, RevB, mv, par, sv, rv, av, pv, y);
+        launchNFFRange<RevB>(0, nI, mv, par, sv, rv, av, pv, y);
         halo.finish();
-        DAB_LAUNCH_NFF_R(nI, nB, RevB, mv, par, sv, rv, av, pv, y);
+        launchNFFRange<RevB>(nI, nB, mv, par, sv, rv, av, pv, y);
         {
             std::vector<HaloItem> it{{av.gUb, 9, 1, nT}};
             if (par.turb) it.push_back({av.gNtb, 3, 1, nT});
             halo.start(halo.cells, it);
         }
-        DAB_LAUNCH_NF_R(0, nI, RevC, mv, par, sv, rv, av, y, 0);
+        launchNFRange<RevC>(0, nI, mv, par, sv, rv, av, y, 0);
         halo.finish();
-        DAB_LAUNCH_NF_R(nI, nB, RevC, mv, par, sv, rv, av, y, 0);
+        launchNFRange<RevC>(nI, nB, mv, par, sv, rv, av, y, 0);
     }
 
     // ghost values of the input vector, exchange started but not awaited (halo.finish() before the first reader)
@@ -1769,32 +1545,18 @@ struct Solver
         if (par.comp)
         {
             // DARhoSimpleFoam: 0 cRevA, 1 cRevB, 2 cRevE + cRevC
-            if (which == 0) DAB_LAUNCH_NF(hm.nC, cRevA, mv, par, sv, rv, av, pv);
-            else if (which == 1) DAB_LAUNCH_NF(hm.nC, cRevB, mv, par, sv, rv, av, pv, dY2.p);
+            if (which == 0) launchNF<cRevA>(hm.nC, mv, par, sv, rv, av, pv);
+            else if (which == 1) launchNF<cRevB>(hm.nC, mv, par, sv, rv, av, pv, dY2.p);
             else
             {
-                DAB_LAUNCH_NF(hm.nC, cRevE, mv, par, sv, rv, av, pv, dY2.p);
-                DAB_LAUNCH_NF(hm.nC, cRevC, mv, par, sv, rv, av, dY2.p);
+                launchNF<cRevE>(hm.nC, mv, par, sv, rv, av, pv, dY2.p);
+                launchNF<cRevC>(hm.nC, mv, par, sv, rv, av, dY2.p);
             }
             return;
         }
-        if (tileProduct())
-        {
-            // tile kernels: 0 = RevA tile, 1 = fused RevB+RevC tile (there is no separate RevC)
-            if (which == 0) launchTileA(pv);
-            else if (which == 1) launchTileBC(pv, dY2.p);
-            return;
-        }
-        if (ghosted())
-        {
-            if (which == 0) launchRevA(pv);
-            else if (which == 1) DAB_LAUNCH_NFF(hm.nC, RevB, mv, par, sv, rv, av, pv, dY2.p);
-            else DAB_LAUNCH_NF(hm.nC, RevC, mv, par, sv, rv, av, dY2.p, 0);
-            return;
-        }
-        if (which == 0) DAB_LAUNCH_NF_PF(pfRevA(pv), hm.nC, RevA, mv, par, sv, rv, av, pv);
-        else if (which == 1) DAB_LAUNCH_NFF_PF(pfRevB(pv), hm.nC, RevB, mv, par, sv, rv, av, pv, dY2.p);
-        else DAB_LAUNCH_NF_PF(pfRevC(), hm.nC, RevC, mv, par, sv, rv, av, dY2.p, 0);
+        if (which == 0) launchNF<RevA>(hm.nC, mv, par, sv, rv, av, pv);
+        else if (which == 1) launchNFF<RevB>(hm.nC, mv, par, sv, rv, av, pv, dY2.p);
+        else launchNF<RevC>(hm.nC, mv, par, sv, rv, av, dY2.p, 0);
     }
 
     void matVec(const double* x, double* y)
@@ -2162,9 +1924,9 @@ struct Solver
                 be.zero(av.gPb, (size_t)3 * hm.nCtot * sizeof(double));
                 be.zero(av.gNtb, (size_t)3 * hm.nCtot * sizeof(double));
                 be.zero(av.gHeb, (size_t)3 * hm.nCtot * sizeof(double));
-                DAB_LAUNCH_NF(hm.nC, cForceRevA, mv, par, sv, rv, av, specs[g], seed);
+                launchNF<cForceRevA>(hm.nC, mv, par, sv, rv, av, specs[g], seed);
                 if (ghosted()) halo.exchangeCells({{av.gUb, 9, 1, hm.nCtot}});
-                DAB_LAUNCH_NF(hm.nC, cRevC, mv, par, sv, rv, av, dY2.p);
+                launchNF<cRevC>(hm.nC, mv, par, sv, rv, av, dY2.p);
                 be.zero(dY2.p + (size_t)nCellStates() * hm.nC, (size_t)hm.nF * sizeof(double)); // no face-flux dependence
                 if (g == 0)
                     be.d2h(out, dY2.p, (size_t)nDof() * sizeof(double));
@@ -2181,13 +1943,13 @@ struct Solver
         be.zero(av.gUb, (size_t)9 * hm.nCtot * sizeof(double));
         be.zero(av.gPb, (size_t)3 * hm.nCtot * sizeof(double));
         be.zero(av.gNtb, (size_t)3 * hm.nCtot * sizeof(double));
-        DAB_LAUNCH_NF(hm.nC, ForceRevA, mv, par, sv, rv, av, forceSpec(f), seed);
+        launchNF<ForceRevA>(hm.nC, mv, par, sv, rv, av, forceSpec(f), seed);
         if (ghosted())
         {
             std::vector<HaloItem> it{{av.gUb, 9, 1, hm.nCtot}};
             halo.exchangeCells(it);
         }
-        DAB_LAUNCH_NF(hm.nC, RevC, mv, par, sv, rv, av, dY2.p, 1);
+        launchNF<RevC>(hm.nC, mv, par, sv, rv, av, dY2.p, 1);
         be.d2h(out, dY2.p, (size_t)nDof() * sizeof(double));
     }
 

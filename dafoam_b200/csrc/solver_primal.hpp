@@ -279,7 +279,7 @@ inline int Solver::solvePrimal(PrimalStats& st)
     Params pp = par; // the primal kernels see the stored, relaxed density
     if (par.comp)
     {
-        DAB_LAUNCH_NF(nT, cFwdA, mv, par, sv, rv); // rho = psi*p of the initial state (ghost cells included)
+        launchNF<cFwdA>(nT, mv, par, sv, rv); // rho = psi*p of the initial state (ghost cells included)
         pp.rhoFrozen = 1;
     }
     for (it = 1; par.comp && it <= P.maxIters; it++)
@@ -287,9 +287,9 @@ inline int Solver::solvePrimal(PrimalStats& st)
         // ---- DARhoSimpleFoam: UEqnRhoSimple.H, EEqnRhoSimple.H, pEqnRhoSimple.H, turbulence.correct()
         maxRes = -1e10;
         be.d2d(P.pOld.p, dP.p, (size_t)nT * sizeof(double));
-        DAB_LAUNCH_NF(nT, cFwdA, mv, pp, sv, rv);
+        launchNF<cFwdA>(nT, mv, pp, sv, rv);
         exGrad();
-        DAB_LAUNCH_NF(nC, cUEqnAssemble, mv, pp, sv, rv, eU);
+        launchNF<cUEqnAssemble>(nC, mv, pp, sv, rv, eU);
         primalJacobi(eU, dU.p, P.Utmp.p, rv.gP, P.cU, st.resU);
         {
             double s3[3] = {st.resU[0], st.resU[1], st.resU[2]};
@@ -297,9 +297,9 @@ inline int Solver::solvePrimal(PrimalStats& st)
             maxRes = std::max(maxRes, s3[1]);
         }
         // energy: solve for he, T from he (thermo.correct())
-        DAB_LAUNCH_NF(nT, cFwdA, mv, pp, sv, rv);
+        launchNF<cFwdA>(nT, mv, pp, sv, rv);
         exGrad();
-        DAB_LAUNCH_NF(nC, cEEqnAssemble, mv, pp, sv, rv, eE, P.alphaE);
+        launchNF<cEEqnAssemble>(nC, mv, pp, sv, rv, eE, P.alphaE);
         {
             double re[3];
             primalJacobi(eE, rv.he, P.heTmp.p, nullptr, P.cE, re);
@@ -310,7 +310,7 @@ inline int Solver::solvePrimal(PrimalStats& st)
             if (mr) halo.exchangeCells({{dT.p, 1, 1, nT}});
         }
         // pressure corrector
-        DAB_LAUNCH_NF(nT, cFwdA, mv, pp, sv, rv);
+        launchNF<cFwdA>(nT, mv, pp, sv, rv);
         exGrad();
         be.launch(nC, HbyAKernel{eU, sv, rv, mv.V, nT});
         if (mr) halo.exchangeCells({{rv.rAU, 1, 1, nT}, {rv.HbyA, 3, 1, nT}});
@@ -322,7 +322,7 @@ inline int Solver::solvePrimal(PrimalStats& st)
             be.d2d(P.gPOld.p, rv.gP, (size_t)3 * nT * sizeof(double));
             sc = Simplec{P.rAt.p, P.pOld.p, P.gPOld.p};
         }
-        DAB_LAUNCH_NF(nC, cPEqnAssemble, mv, pp, sv, rv, eP, sc);
+        launchNF<cPEqnAssemble>(nC, mv, pp, sv, rv, eP, sc);
         if (it == 1 || (it - 1) % P.coarseRefresh == 0) primalCoarseRefresh(eP);
         {
             double rp;
@@ -331,22 +331,22 @@ inline int Solver::solvePrimal(PrimalStats& st)
             maxRes = std::max(maxRes, rp);
         }
         if (mr) halo.exchangeCells({{dP.p, 1, 1, nT}});
-        DAB_LAUNCH_NF(nC, cPhiUpdate, mv, pp, sv, rv, dPhi.p, sc);
+        launchNF<cPhiUpdate>(nC, mv, pp, sv, rv, dPhi.p, sc);
         if (mr) halo.exchangeFaces({{dPhi.p, 1, 1, hm.nF}});
         be.launch(nC, RelaxField{dP.p, P.pOld.p, P.alphaP});
         be.launch(nC, BoundField{dP.p, P.pMin, P.pMax});
         be.launch(nC, RhoRelax{pp, sv, rv.rho, P.alphaRho});
         if (mr) halo.exchangeCells({{dP.p, 1, 1, nT}, {rv.rho, 1, 1, nT}});
-        DAB_LAUNCH_NF(nT, cFwdA, mv, pp, sv, rv); // grad of the relaxed p, closures at the new (p, T)
+        launchNF<cFwdA>(nT, mv, pp, sv, rv); // grad of the relaxed p, closures at the new (p, T)
         exGrad();
         be.launch(nC, UCorrect{rv, dU.p, nT, sc});
         be.launch(3 * nC, BoundField{dU.p, -P.UMax, P.UMax});
         if (mr) halo.exchangeCells({{dU.p, 3, 3, 1}});
         if (par.turb)
         {
-            DAB_LAUNCH_NF(nT, cFwdA, mv, pp, sv, rv);
+            launchNF<cFwdA>(nT, mv, pp, sv, rv);
             exGrad();
-            DAB_LAUNCH_NF(nC, cNutEqnAssemble, mv, pp, sv, rv, eN, P.alphaN);
+            launchNF<cNutEqnAssemble>(nC, mv, pp, sv, rv, eN, P.alphaN);
             double rn[3];
             primalJacobi(eN, dNt.p, P.ntTmp.p, nullptr, P.cN, rn);
             st.resN = rn[0];
@@ -365,9 +365,9 @@ inline int Solver::solvePrimal(PrimalStats& st)
         maxRes = -1e10;
         be.d2d(P.pOld.p, dP.p, (size_t)nT * sizeof(double)); // p.storePrevIter()
         // --- momentum predictor (UEqnSimple.H)
-        DAB_LAUNCH_NF(nT, FwdA, mv, par, sv, rv);
+        launchNF<FwdA>(nT, mv, par, sv, rv);
         exGrad();
-        DAB_LAUNCH_NFF(nC, UEqnAssemble, mv, par, sv, rv, eU);
+        launchNFF<UEqnAssemble>(nC, mv, par, sv, rv, eU);
         primalJacobi(eU, dU.p, P.Utmp.p, rv.gP, P.cU, st.resU);
         {
             double s3[3] = {st.resU[0], st.resU[1], st.resU[2]};
@@ -389,10 +389,10 @@ inline int Solver::solvePrimal(PrimalStats& st)
         {
             if (no > 0)
             {
-                DAB_LAUNCH_NF(nT, FwdA, mv, par, sv, rv); // grad(p) of the latest p for the non-orthogonal correction
+                launchNF<FwdA>(nT, mv, par, sv, rv); // grad(p) of the latest p for the non-orthogonal correction
                 exGrad();
             }
-            DAB_LAUNCH_NF(nC, PEqnAssemble, mv, par, sv, rv, eP, sc);
+            launchNF<PEqnAssemble>(nC, mv, par, sv, rv, eP, sc);
             if (no == 0 && (it == 1 || (it - 1) % P.coarseRefresh == 0)) primalCoarseRefresh(eP);
             double rp;
             st.pIterations += primalPcg(eP, dP.p, P.cP, rp);
@@ -400,20 +400,20 @@ inline int Solver::solvePrimal(PrimalStats& st)
             maxRes = std::max(maxRes, rp);
         }
         if (mr) halo.exchangeCells({{dP.p, 1, 1, nT}});
-        DAB_LAUNCH_NF(nC, PhiUpdate, mv, par, sv, rv, dPhi.p, sc);
+        launchNF<PhiUpdate>(nC, mv, par, sv, rv, dPhi.p, sc);
         if (mr) halo.exchangeFaces({{dPhi.p, 1, 1, hm.nF}}); // cut faces: the owner rank's flux
         be.launch(nC, RelaxField{dP.p, P.pOld.p, P.alphaP});
         if (mr) halo.exchangeCells({{dP.p, 1, 1, nT}});
-        DAB_LAUNCH_NF(nT, FwdA, mv, par, sv, rv); // grad of the relaxed p
+        launchNF<FwdA>(nT, mv, par, sv, rv); // grad of the relaxed p
         exGrad();
         be.launch(nC, UCorrect{rv, dU.p, nT, sc});
         if (mr) halo.exchangeCells({{dU.p, 3, 3, 1}});
         // --- turbulence (DASpalartAllmaras::correct)
         if (par.turb)
         {
-            DAB_LAUNCH_NF(nT, FwdA, mv, par, sv, rv);
+            launchNF<FwdA>(nT, mv, par, sv, rv);
             exGrad();
-            DAB_LAUNCH_NF(nC, NutEqnAssemble, mv, par, sv, rv, eN, P.alphaN);
+            launchNF<NutEqnAssemble>(nC, mv, par, sv, rv, eN, P.alphaN);
             double rn[3];
             primalJacobi(eN, dNt.p, P.ntTmp.p, nullptr, P.cN, rn);
             st.resN = rn[0];

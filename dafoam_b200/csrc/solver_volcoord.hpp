@@ -201,12 +201,12 @@ inline void Solver::volCoordProduct(const double* psi, const FunctionDef* functi
         {
             if (par.comp)
             {
-                DAB_LAUNCH_NF(hm.nCtot, cFwdA, mv, par, sv, rv);
+                launchNF<cFwdA>(hm.nCtot, mv, par, sv, rv);
                 for (const ForceSpec& fs : fsv) be.launch(hm.nBF, cForceFwd{mv, par, sv, rv, fs, Fdev});
             }
             else
             {
-                DAB_LAUNCH_NF(hm.nCtot, FwdA, mv, par, sv, rv);
+                launchNF<FwdA>(hm.nCtot, mv, par, sv, rv);
                 for (const ForceSpec& fs : fsv) be.launch(hm.nBF, ForceFwd{mv, par, sv, rv, fs, Fdev});
             }
         }

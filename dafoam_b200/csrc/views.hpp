@@ -285,11 +285,10 @@ DAB_HD FaceRef faceOfE(const MeshView& m, int e, int n)
     return r;
 }
 
-// DAB_PREFETCH_IDX (default build): load the cell's whole row of the two ELL tables before the face loop (fixed-size
-// meshes), so that the index loads of all faces are in flight together instead of one dependent round trip per face
-// (measured on B200: product 0.855 -> 0.763 ms).  Requesting the NEXT face's cache lines with prefetch.global.L1 on top of
-// this was measured too and is slower (1.005 ms: the prefetches double the LSU transactions) -- not kept.
-#if defined(DAB_PREFETCH_IDX)
+// load the cell's whole row of the two ELL tables before the face loop (fixed-size meshes), so that the index loads of all
+// faces are in flight together instead of one dependent round trip per face (measured on B200: product 0.855 -> 0.763 ms).
+// Requesting the NEXT face's cache lines with prefetch.global.L1 on top of this was measured too and is slower (1.005 ms:
+// the prefetches double the LSU transactions) -- not kept.
 #define DAB_FACE_PREFETCH(NF)                                                                    \
     int e_[(NF) > 0 ? (NF) : 1], n_[(NF) > 0 ? (NF) : 1];                                        \
     if ((NF) > 0)                                                                                \
@@ -301,10 +300,6 @@ DAB_HD FaceRef faceOfE(const MeshView& m, int e, int n)
         }                                                                                        \
     }
 #define DAB_FACE(NF, k) ((NF) > 0 ? faceOfE(m, e_[(NF) > 0 ? (k) : 0], n_[(NF) > 0 ? (k) : 0]) : faceOf(m, c, k))
-#else
-#define DAB_FACE_PREFETCH(NF)
-#define DAB_FACE(NF, k) faceOf(m, c, k)
-#endif
 
 // SA constants (reference src/adjoint/DAModel/DATurbulenceModel/DASpalartAllmaras.C:47-80)
 struct SA

@@ -19,8 +19,6 @@ d = tempfile.mkdtemp(prefix="dab_kb_")
 cases.write_case(d, mesh, cases.default_bcs_naca(), binary=True)
 for lib in libs:
     opts = dict(normalizeStates=dict(U=10.0, p=50.0, nuTilda=1e-3, phi=1.0))
-    if tile:
-        opts["adjEqnOption"] = dict(tileCells=int(np.prod([int(v) for v in tile.split("x")])))
     sol = pyDASolvers("DASimpleFoam -python", opts, caseDir=d, _lib_path=lib)
     n = sol.getNLocalAdjointStates()
     y = np.zeros(sol.getNLocalCells()); sol.getOFField("yWall", "scalar", y)

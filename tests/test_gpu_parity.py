@@ -96,30 +96,3 @@ def test_values_match_the_oracle_on_a_34k_cell_mesh_cuda():
     for a, b in ((0, 3 * nC), (3 * nC, 4 * nC), (4 * nC, 5 * nC), (5 * nC, orc.ndof)):
         assert rel_err(y[a:b], yo[a:b]) < 1e-10
 
-
-def test_tile_kernels_match_the_default_kernels_cuda():
-    """DAB_TILE=1 (CTA-resident tile kernels, chosen once per process: child processes) computes the same product as the default
-    cell-per-thread kernels on a tile-major numbered mesh with real halos."""
-    import os, subprocess, sys
-    code = r'''
-import numpy as np, sys
-from tests.test_gpu_parity import _medium_case
-mesh, orc, sol, W = _medium_case(160, 96, extra=dict(adjEqnOption=dict(tileCells=192)))
-sol.updateOFFields(W)
-psi = np.random.default_rng(7).uniform(-1, 1, orc.ndof)
-y = np.zeros(orc.ndof)
-sol.calcdRdWTPsiAD(psi, y)
-np.save(sys.argv[1], y)
-'''
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = {}
-    import tempfile
-    for tile in ("0", "1"):
-        f = os.path.join(tempfile.mkdtemp(), "y.npy")
-        r = subprocess.run([sys.executable, "-c", code, f], cwd=root, env=dict(os.environ, DAB_TILE=tile, PYTHONPATH=root, DAB_TILE_INFO="1"),
-                           capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        if tile == "1":
-            assert "tiles: 192 cells per tile" in r.stderr
-        out[tile] = np.load(f)
-    assert rel_err(out["1"], out["0"]) < 1e-12
